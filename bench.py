@@ -7,6 +7,8 @@ A "step" = one closed burst of (64 x n_gpus) chat-completion requests through th
 K1 admission (rpm/tpm debit + least-busy pick) -> per-GPU engine: chunked prefill + 127 decode steps
 (CUDA graph) -> DONE events.  Launch:  python bench.py --gpus N --steps K --warmup W
 (N > 1: python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...).
+Inputs (weights, prompts) are seeded: --dump-outputs DIR stores what the last timed burst returned (generated tokens, router
+picks) as .npy, so that two builds can be compared output for output.
 
   value      completions/s from device time only: CUDA events on each engine's stream around every
              prefill chunk and every decode step of the timed steps (inputs resident), max over ranks.
@@ -65,7 +67,13 @@ def parse_args():
     ap.add_argument("--config", default="headline", choices=sorted(CONFIGS),
                     help="BASELINE.json config: headline (#1, default), quota (#2), fallback (#3), fleet (#4)")
     ap.add_argument("--trace-out", default=None, help="fleet configs: write the recorded admission trace here (JSON)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="headline config: after the timed steps write what the last one returned to its callers as DIR/*.npy "
+                         "(float32): tokens [requests, max_new] = generated token ids, deployment [requests] = router pick")
+    args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "b200" or CONFIGS[args.config] != "headline"):
+        ap.error("--dump-outputs applies to the headline config of --impl b200")
+    return args
 
 
 def load_peaks():
@@ -491,11 +499,13 @@ def main():
 
     ttfts, lat = [], []
     token_sums = []                                                # per step: checksum of every generated token
+    last = {}                                                      # what the latest burst returned (--dump-outputs)
 
     def one_step(collect: bool):
         """One closed burst through the public path.  Returns nothing; per-request timings collected."""
         if world == 1:
             out = router.completion_batch(args.model, [prompts_np[i] for i in range(n_req)], M)
+            last["out"] = out
             chk = 0
             for i, r in enumerate(out):
                 if isinstance(r, Exception):
@@ -515,6 +525,7 @@ def main():
             ids = np.ascontiguousarray(prompts_np[mine]).reshape(-1)
             start = np.arange(0, (len(mine) + 1) * P, P, dtype=np.int32)
             recs, _ = eng.run_batch(ids, start, M) if len(mine) else ([], None)
+            last["out"] = (mine, recs, dec)
             assert all(r.status == 0 and len(r.tokens) == M for r in recs)
             # checksum keyed by REQUEST (which rank serves a request may change from burst to burst: least-busy ties are
             # broken through the router's RNG stream), summed over the ranks
@@ -554,6 +565,26 @@ def main():
     # identical prompts every step and deterministic kernels: every step must have generated exactly the same tokens for
     # every request
     assert len(set(token_sums)) == 1, "generated tokens differ between bursts"
+    if args.dump_outputs:
+        # the last timed burst as its callers received it, by request id; token ids < 2^24 are exact in float32
+        tok, dep = np.zeros((n_req, M)), np.zeros(n_req)
+        if world == 1:
+            for i, r in enumerate(last["out"]):
+                tok[i], dep[i] = r._token_ids, r._deployment
+        else:
+            mine, recs, dec = last["out"]
+            for i, r in zip(mine, recs):
+                tok[i] = r.tokens
+            if rank == 0:
+                dep[:] = [d[1] for d in dec]
+            both = torch.from_numpy(np.concatenate([tok.ravel(), dep])).to(f"cuda:{local}")
+            dist.all_reduce(both, op=dist.ReduceOp.SUM)                # each request's row is filled on one rank only
+            both = both.cpu().numpy()
+            tok, dep = both[: n_req * M].reshape(n_req, M), both[n_req * M:]
+        if rank == 0:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            np.save(os.path.join(args.dump_outputs, "tokens.npy"), tok.astype(np.float32))
+            np.save(os.path.join(args.dump_outputs, "deployment.npy"), dep.astype(np.float32))
 
     # ---- max over ranks
     vals = torch.tensor([wall, dev_s, st["decode_ms_total"], float(st["decode_steps"]), st["prefill_ms_total"],

@@ -1,145 +1,171 @@
-"""CPU: the reference's three gateway demo scripts, UNMODIFIED, run as subprocesses against this repo's HTTP gateway
-(sample-resilient-llm-inference_b200/server.py) -- cwd holds ./config/config.yaml exactly as the scripts expect
-(reference src/demo_fallback.py:16, src/demo_load_balancing.py:20, src/demo_quota_isolation.py:19).
+"""CPU: the traffic of the reference's three gateway demo scripts (reference src/demo_fallback.py,
+src/demo_load_balancing.py, src/demo_quota_isolation.py) against this repo's HTTP gateway
+(sample-resilient-llm-inference_b200/server.py), sent with the OpenAI SDK the scripts use.
 
-The router kernel needs a GPU and /root/reference does not exist on the GPU box, so this test puts a RECORDING DOUBLE behind
-server.py (first-fit over the config's rpm limits -- a test double, not the product and not the oracle): what it proves is
-the wire contract -- the scripts' OpenAI-SDK calls are served, `.model` / HTTP 429 are understood by their exception
-handling, their own end-of-run tables come out with the README's counts (reference README.md:167-171, 206-213, 262-264).
-Every request they make is recorded into tests/golden/reference_demo_requests.json; tests/test_reference_demos_gpu.py
-replays exactly those requests against the real K1-backed gateway on the B200.
-Regenerate the fixture:  RR_WRITE_GOLDEN=1 python -m pytest tests/test_reference_demos_cpu.py"""
+The router kernel needs a GPU, so a RECORDING DOUBLE sits behind server.py (first-fit over the config's rpm limits -- a
+test double, not the product and not the oracle): what this proves is the wire contract -- the scripts' OpenAI-SDK calls
+are served, `.model` / HTTP 429 are understood by their exception handling, and their end-of-run tables come out with the
+README's counts (reference README.md:167-171, 206-213, 262-264).
+
+tests/golden/make_demo_golden.py ran the UNMODIFIED scripts against this gateway and stored in
+tests/golden/reference_demo_wire.json every request they sent (SDK retries included), what the double answered, and the
+figures the scripts printed at the end.  This test issues the same calls the way the scripts issue them (one thread per
+request, their stagger and timeout, a shared client or one client per request, the SDK's default retries) and checks that
+the gateway receives the same requests, answers them the same way, and that the scripts' own tallying of the responses
+gives the recorded figures.  tests/test_reference_demos_gpu.py replays the distinct requests
+(tests/golden/reference_demo_requests.json) against the real K1-backed gateway on the B200."""
 import json
 import os
-import re
-import shutil
 import socket
-import subprocess
-import sys
 import threading
 import time
-
-import pytest
+from collections import Counter
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference/src"
+CFG = os.path.join(ROOT, "config", "config.yaml")
+WIRE = os.path.join(ROOT, "tests", "golden", "reference_demo_wire.json")
 GOLD = os.path.join(ROOT, "tests", "golden", "reference_demo_requests.json")
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="the reference tree is only present in the build container")
+
+# how each script issues its requests: seconds between thread starts, one OpenAI client per request, request timeout
+# (src/demo_fallback.py:28,146,216; src/demo_load_balancing.py:24,109,199; src/demo_quota_isolation.py:42,55,135)
+CALLS = {"demo_fallback": (0.05, False, 30), "demo_load_balancing": (0.1, False, 30), "demo_quota_isolation": (0.0, True, 10)}
 
 
 class RecordingDouble:
-    """First-fit admission over the YAML's rpm limits + fallbacks; records every request."""
+    """First-fit admission over the YAML's rpm limits + fallbacks; records every request and its answer."""
 
     def __init__(self, cfg):
         from rr_b200.router import Choice, Message, ModelResponse, RateLimitError, BadRequestError, Usage
         self.cfg, self.used, self.log, self.lock = cfg, [0] * len(cfg.deployments), [], threading.Lock()
         self._t = (Choice, Message, ModelResponse, RateLimitError, BadRequestError, Usage)
 
+    def _admit(self, model):
+        g = self.cfg.group_index(model)
+        if g < 0:
+            return 400
+        for grp in [g] + self.cfg.fallbacks.get(g, []):
+            for d in self.cfg.deployments:
+                if d.group == grp and (d.rpm < 0 or self.used[d.index] < d.rpm):
+                    self.used[d.index] += 1
+                    return d.response_model
+        return 429
+
     def completion(self, model, messages, timeout=None, max_tokens=None):
         Choice, Message, ModelResponse, RateLimitError, BadRequestError, Usage = self._t
         with self.lock:
-            self.log.append({"model": model, "messages": messages, "timeout": timeout})
-            g = self.cfg.group_index(model)
-            if g < 0:
-                raise BadRequestError(f"Invalid model name passed in model={model}")
-            for grp in [g] + self.cfg.fallbacks.get(g, []):
-                for d in self.cfg.deployments:
-                    if d.group == grp and (d.rpm < 0 or self.used[d.index] < d.rpm):
-                        self.used[d.index] += 1
-                        return ModelResponse("chatcmpl-double", d.response_model, [Choice(0, Message("assistant", "ok"))], Usage(8, 2, 10))
+            outcome = self._admit(model)
+            self.log.append({"model": model, "messages": messages, "outcome": outcome})
+        if outcome == 400:
+            raise BadRequestError(f"Invalid model name passed in model={model}")
+        if outcome == 429:
             raise RateLimitError(f"No deployments available for selected model, passed model={model}")
+        return ModelResponse("chatcmpl-double", outcome, [Choice(0, Message("assistant", "ok"))], Usage(8, 2, 10))
 
     def snapshot(self):
         return []
 
 
-def _free_port():
-    s = socket.socket(); s.bind(("127.0.0.1", 0)); p = s.getsockname()[1]; s.close()
-    return p
-
-
-def _run_demo(script, tmp_path, args=()):
+def serve_double(host="127.0.0.1"):
+    """server.py in front of a fresh RecordingDouble on a free port -> (double, uvicorn server, thread, port)."""
     import uvicorn
-    import yaml
     from rr_b200.config import load_config
     from rr_b200.server import create_app
-    port = _free_port()
-    os.makedirs(tmp_path / "config", exist_ok=True)
-    with open(os.path.join(ROOT, "config", "config.yaml")) as f:
-        raw = yaml.safe_load(f)
-    raw["litellm"]["port"] = port                                   # the scripts read the port from ./config/config.yaml
-    with open(tmp_path / "config" / "config.yaml", "w") as f:
-        yaml.safe_dump(raw, f)
-    dbl = RecordingDouble(load_config(str(tmp_path / "config" / "config.yaml")))
-    server = uvicorn.Server(uvicorn.Config(create_app(dbl), host="0.0.0.0", port=port, log_level="error"))
+    s = socket.socket(); s.bind(("127.0.0.1", 0)); port = s.getsockname()[1]; s.close()
+    dbl = RecordingDouble(load_config(CFG))
+    server = uvicorn.Server(uvicorn.Config(create_app(dbl), host=host, port=port, log_level="error"))
     th = threading.Thread(target=server.run, daemon=True)
     th.start()
     for _ in range(200):
         if server.started:
             break
         time.sleep(0.05)
-    try:
-        env = dict(os.environ, PYTHONUNBUFFERED="1", NO_COLOR="1")
-        p = subprocess.run([sys.executable, os.path.join(REF, script), *args], cwd=str(tmp_path), env=env, capture_output=True,
-                           text=True, timeout=180)
-    finally:
-        server.should_exit = True
-        th.join(10)
-    out = re.sub(r"\x1b\[[0-9;]*m", "", p.stdout)
-    assert p.returncode == 0, (p.returncode, out[-2000:], p.stderr[-2000:])
-    return out, dbl.log
+    return dbl, server, th, port
 
 
-def _num(out, label):
-    m = re.search(re.escape(label) + r"\s*:?\s*(\d+)", out)
-    assert m, (label, out[-1500:])
-    return int(m.group(1))
+def tally(demo, calls, got):
+    """The end-of-run figures of a demo script, counted its way from the responses (`.model`, or 429 / another error)."""
+    ok = [g for g in got if isinstance(g, str)]
+    if demo == "demo_fallback":                                     # src/demo_fallback.py:154,227-230
+        fb = sum("sonnet-3-5" in g.lower() or "3-5-sonnet" in g.lower() for g in ok)
+        return {"total": len(got), "successful": len(ok), "failed": len(got) - len(ok), "primary": len(ok) - fb, "fallback": fb}
+    if demo == "demo_load_balancing":                               # src/demo_load_balancing.py:192,210-222
+        return {"total": len(got), "successful": len(ok), "failed": len(got) - len(ok), "distribution": dict(Counter(ok))}
+    rows = {}                                                       # src/demo_quota_isolation.py:241-243
+    for c, g in zip(calls, got):
+        r = rows.setdefault(c["model"].split("-")[1].upper(), [0, 0, 0, 0])   # consumer-a-model -> A
+        r[0] += 1; r[1] += isinstance(g, str); r[2] += not isinstance(g, str); r[3] += g == 429
+    return {"rows": rows}
 
 
-def test_unmodified_reference_demos_against_this_gateway(tmp_path):
-    recorded = {}
-    # ---- fallback demo: 10 concurrent requests, primary rpm 3 -> 3 primary + 7 fallback (README.md:167-171)
-    out, log = _run_demo("demo_fallback.py", tmp_path / "fb")
-    assert _num(out, "Total Requests") == 10 and _num(out, "Successful") == 10 and _num(out, "Failed") == 0
-    assert _num(out, "Primary Model Used") == 3 and _num(out, "Fallback Triggered") == 7
-    recorded["demo_fallback"] = log
-    # ---- load-balancing demo: 3 + 3 on the two primaries, 4 on the fallback (README.md:206-213)
-    out, log = _run_demo("demo_load_balancing.py", tmp_path / "lb")
-    assert len(log) == 10 and all(r["model"] == "claude-sonnet-loadbalance-demo" for r in log)
-    counts = sorted(int(c) for c in re.findall(r":\s+(\d+) requests", out))
-    assert counts[-3:] == [3, 3, 4] or sum(counts) >= 10, out[-1500:]
-    recorded["demo_load_balancing"] = log
-    # ---- quota isolation: A 3/5 (2 rate limited), B 5/5, C 5/5 (README.md:262-264)
-    out, log = _run_demo("demo_quota_isolation.py", tmp_path / "q")
-    by, attempts = {}, {}
-    for r in log:
-        by.setdefault(r["model"], set()).add(r["messages"][0]["content"])
-        attempts[r["model"]] = attempts.get(r["model"], 0) + 1
-    assert {k: len(v) for k, v in by.items()} == {"consumer-a-model": 5, "consumer-b-model": 5, "consumer-c-model": 5}
-    # the OpenAI SDK retries a 429 twice by default (one client per request, reference src/demo_quota_isolation.py:42):
-    # team A's two rejected requests arrive three times each
-    assert attempts == {"consumer-a-model": 9, "consumer-b-model": 5, "consumer-c-model": 5}
-    rows = {m.group(1): tuple(int(x) for x in m.group(2, 3, 4, 5))
-            for m in re.finditer(r"^([ABC])\s+\|\s+\w+\s+\|\s+[\d.]+%\s+\|\s+(\d+) \|\s+(\d+) \|\s+(\d+) \|\s+(\d+) \|", out, re.M)}
-    # the script's own table: (total, success, failed, rate limited) per consumer
-    assert rows == {"A": (5, 3, 2, 2), "B": (5, 5, 0, 0), "C": (5, 5, 0, 0)}, (rows, out[-1500:])
-    recorded["demo_quota_isolation"] = log
-    # every call has the shape SURVEY.md 8b states: model (group name), one user message, a timeout
-    for name, log in recorded.items():
-        for r in log:
-            assert isinstance(r["model"], str) and len(r["messages"]) == 1 and r["messages"][0]["role"] == "user"
-    slim = {}
-    for k, v in recorded.items():                                  # distinct requests (SDK retries folded), arrival order
-        seen, lst = set(), []
-        for r in v:
-            key_ = (r["model"], r["messages"][0]["content"])
-            if key_ not in seen:
-                seen.add(key_); lst.append({"model": key_[0], "content": key_[1]})
-        slim[k] = lst
-    if os.environ.get("RR_WRITE_GOLDEN") or not os.path.exists(GOLD):
-        with open(GOLD, "w") as f:
-            json.dump(slim, f, indent=1, sort_keys=True)
+def distinct_calls(wire):
+    """The client calls behind a recorded request stream: SDK retries folded, first-arrival order."""
+    seen, out = set(), []
+    for r in wire:
+        key = (r["model"], json.dumps(r["messages"]))
+        if key not in seen:
+            seen.add(key); out.append({"model": r["model"], "messages": r["messages"]})
+    return out
+
+
+def _replay(port, calls, stagger, per_request, timeout):
+    import openai
+    shared = openai.OpenAI(api_key="demo-key", base_url=f"http://127.0.0.1:{port}")
+    got = [None] * len(calls)
+
+    def work(i, c):
+        client = openai.OpenAI(api_key=f"key-{i}", base_url=f"http://127.0.0.1:{port}") if per_request else shared
+        try:
+            got[i] = getattr(client.chat.completions.create(model=c["model"], messages=c["messages"], timeout=timeout), "model", "unknown")
+        except openai.RateLimitError:
+            got[i] = 429
+        except Exception as e:                                      # noqa: BLE001  (a failed request, as the scripts count it)
+            got[i] = repr(e)
+    ths = []
+    for i, c in enumerate(calls):
+        t = threading.Thread(target=work, args=(i, c))
+        t.start(); ths.append(t)
+        if stagger:
+            time.sleep(stagger)
+    for t in ths:
+        t.join()
+    return got
+
+
+def test_recorded_reference_demo_traffic_against_this_gateway():
+    with open(WIRE) as f:
+        rec = json.load(f)
+    assert sorted(rec) == sorted(CALLS)
+    # the scripts' recorded end-of-run figures are the README's
+    assert rec["demo_fallback"]["printed"] == {"total": 10, "successful": 10, "failed": 0, "primary": 3, "fallback": 7}
+    lb = rec["demo_load_balancing"]["printed"]
+    assert lb["total"] == lb["successful"] == 10 and sorted(lb["distribution"].values()) == [3, 3, 4]
+    assert rec["demo_quota_isolation"]["printed"] == {"rows": {"A": [5, 3, 2, 2], "B": [5, 5, 0, 0], "C": [5, 5, 0, 0]}}
+    for demo, (stagger, per_request, timeout) in CALLS.items():
+        wire = rec[demo]["wire"]
+        calls = distinct_calls(wire)
+        # every call has the shape SURVEY.md 8b states: model (group name), one user message
+        assert all(len(c["messages"]) == 1 and c["messages"][0]["role"] == "user" for c in calls)
+        dbl, server, th, port = serve_double()
+        try:
+            got = _replay(port, calls, stagger, per_request, timeout)
+        finally:
+            server.should_exit = True
+            th.join(10)
+        assert tally(demo, calls, got) == rec[demo]["printed"], (demo, got)
+        # the same requests reached the gateway, as often per model group (SDK retries included: a 429 is retried twice,
+        # so team A's two rejected requests arrive three times each; which two lose the race differs from run to run), and
+        # were answered the same way
+        assert sorted(map(json.dumps, distinct_calls(dbl.log))) == sorted(map(json.dumps, calls)), demo
+        assert Counter(r["model"] for r in dbl.log) == Counter(r["model"] for r in wire), demo
+        answers = lambda log: Counter((r["model"], r["outcome"]) for r in log)
+        assert answers(dbl.log) == answers(wire), demo
+    assert Counter(r["model"] for r in rec["demo_quota_isolation"]["wire"]) == {"consumer-a-model": 9, "consumer-b-model": 5,
+                                                                                "consumer-c-model": 5}
+    assert Counter(r["outcome"] for r in rec["demo_quota_isolation"]["wire"])[429] == 6
+    # the GPU replay's fixture holds exactly the distinct requests of the recorded streams
     with open(GOLD) as f:
         gold = json.load(f)
     key = lambda lst: sorted((r["model"], r["content"]) for r in lst)
-    assert {k: key(v) for k, v in gold.items()} == {k: key(v) for k, v in slim.items()}, "fixture drifted: RR_WRITE_GOLDEN=1 to regenerate"
+    assert {k: key(v) for k, v in gold.items()} == \
+        {k: key([{"model": c["model"], "content": c["messages"][0]["content"]} for c in distinct_calls(r["wire"])])
+         for k, r in rec.items()}

@@ -1,5 +1,5 @@
 """GPU: the request streams of the reference's three gateway demos -- recorded from the UNMODIFIED scripts by
-tests/test_reference_demos_cpu.py into tests/golden/reference_demo_requests.json -- replayed over HTTP with the OpenAI SDK
+tests/golden/make_demo_golden.py into tests/golden/reference_demo_requests.json -- replayed over HTTP with the OpenAI SDK
 (the reference's client boundary, src/demo_load_balancing.py:24,106-110) against the real gateway: K1 router kernel +
 config/config.yaml, with mock-completion backends and with tiny real replicas.  Outcomes are the reference README's
 (README.md:167-171: 3 primary + 7 fallback; :206-213: 3 + 3 + 4; :262-264: A 3/5, B 5/5, C 5/5)."""
