@@ -51,7 +51,9 @@ int rr_set_pdl(int enabled);
  * (4 x uint64 each) to `out`. */
 int rr_debug_trace_start(int max_entries);
 int rr_debug_trace_stop(unsigned long long* out, int max_entries, int* n);
-/* on != 0: sample CTAs of the persistent decode layer kernel also record one mark per finished work item (kernel id 12 + phase). */
+/* on = 1: sample CTAs of the fused decode MLP kernel (kernel ids 50 + k) and of the decode attention kernel (80 + k) also
+ * record fixed-slot marks at the end of the trace buffer; on = 10 + s: also those of the plain decode projection with
+ * split-K factor s (100 + k).  on = 0 turns them off. */
 int rr_debug_trace_detail(int on);
 /* Host-side work schedule of the fused decode MLP kernel (gate/up + down GEMMs in one launch, DESIGN.md section 3), for
  * inspection and tests; no device is touched.  items_out receives grid * (*max_items) entries of 4 x int32
@@ -59,12 +61,6 @@ int rr_debug_trace_detail(int on);
  * returns RR_INVALID_ARGUMENT when `capacity` (in entries) is too small (*max_items is still set). */
 int rr_debug_mlp_schedule(int grid, int inter, int hidden, int slice_kb, int32_t* items_out, int capacity,
                           int* max_items);
-
-/* Host-side work schedule of the persistent decode layer kernel (O -> gate/up -> down -> next projection in one launch,
- * DESIGN.md section 3): same entry format with phase 0 = O (slice = split-K plane), 1 = gate/up, 2 = down (slice = K-slice),
- * 3 = next projection (QKV of the next layer / lm_head; slice = split-K plane).  has_main = 0: phase 3 only. */
-int rr_debug_layer_schedule(int grid, int hidden, int inter, int nq, int rows_a3, int s_o, int s3, int slice_kb,
-                            int has_main, int32_t* items_out, int capacity, int* max_items);
 
 /* ================================================================================================
  * 1. Router: admission + rpm/tpm bucket debit + backend pick + cooldown + fallback chain (K1).
@@ -248,7 +244,7 @@ typedef struct rr_engine_opts {
     int32_t use_cuda_graph;       /* capture the decode step */
     int32_t fail_seed;            /* fault injection: seed of the Bernoulli failure mask */
     float fail_prob;              /* fault injection: P(request fails) (BASELINE config #4) */
-    int32_t reserved[4];          /* A/B switches: [0] = 2 persistent decode layer kernel (rr_layer.cu; off by default, measured slower); [1] = 1 no RoPE fusion in the prefill
+    int32_t reserved[4];          /* A/B switches: [0] unused, ignored; [1] = 1 no RoPE fusion in the prefill
                                      QKV epilogue; [2] = 1 no fused decode MLP kernel; [3] = 1 prefill RMSNorm as separate kernels instead of deferred into the GEMM epilogues */
 } rr_engine_opts;
 

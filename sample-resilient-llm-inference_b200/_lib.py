@@ -123,7 +123,6 @@ PROTOTYPES = {
     "rr_debug_trace_detail": (C.c_int, [C.c_int]),
     "rr_debug_trace_stop": (C.c_int, [C.POINTER(C.c_uint64), C.c_int, c_i32p]),
     "rr_debug_mlp_schedule": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, c_i32p, C.c_int, c_i32p]),
-    "rr_debug_layer_schedule": (C.c_int, [C.c_int] * 9 + [c_i32p, C.c_int, c_i32p]),
     "rr_router_create": (C.c_int, [C.POINTER(DeploymentDesc), C.c_int, C.c_int, c_i32p, c_i32p,
                                    C.POINTER(RouterSettings), C.c_uint64, C.c_int,
                                    C.POINTER(vp)]),

@@ -50,8 +50,6 @@ void rr_trace_set_gemm(unsigned long long*);
 void rr_trace_set_attn_decode(unsigned long long*);
 void rr_trace_set_attn_tc(unsigned long long*);
 void rr_trace_set_elementwise(unsigned long long*);
-void rr_trace_set_layer(unsigned long long*);
-void rr_trace_set_layer_detail(int);
 void rr_trace_set_gemm_detail(int);
 void rr_trace_set_attn_decode_detail(int);
 }
@@ -71,7 +69,7 @@ RR_API int rr_debug_trace_start(int max_entries) {
     g_trace_cap = max_entries;
     rr_trace_set_gemm(g_trace_dev); rr_trace_set_attn_decode(g_trace_dev);
     rr_trace_set_attn_tc(g_trace_dev);
-    rr_trace_set_elementwise(g_trace_dev); rr_trace_set_layer(g_trace_dev);
+    rr_trace_set_elementwise(g_trace_dev);
     return check_last();
 }
 // Stops tracing and copies up to max_entries (id, start, dep, end) records; returns the number recorded via *n.
@@ -80,7 +78,7 @@ RR_API int rr_debug_trace_stop(unsigned long long* out, int max_entries, int* n)
     cudaDeviceSynchronize();
     rr_trace_set_gemm(nullptr); rr_trace_set_attn_decode(nullptr);
     rr_trace_set_attn_tc(nullptr);
-    rr_trace_set_elementwise(nullptr); rr_trace_set_layer(nullptr);
+    rr_trace_set_elementwise(nullptr);
     unsigned long long cnt = 0;
     cudaMemcpy(&cnt, g_trace_dev, 8, cudaMemcpyDeviceToHost);
     int m = (int)(cnt < (unsigned long long)g_trace_cap ? cnt : g_trace_cap);
@@ -93,10 +91,9 @@ RR_API int rr_debug_trace_stop(unsigned long long* out, int max_entries, int* n)
     return check_last();
 }
 
-// Per-item marks of sample CTAs inside the persistent layer kernel (tools/trace_layer.py); off by default.
+// Fixed-slot marks of sample CTAs inside the fused MLP / decode attention / plain decode projection kernels; off by default.
 RR_API int rr_debug_trace_detail(int on) {
     g_trace_detail_on = on ? 1 : 0;
-    rr_trace_set_layer_detail(on ? 1 : 0);
     rr_trace_set_gemm_detail(on);      // 1: fused MLP kernel; 10 + s: the plain decode projection with split-K factor s
     rr_trace_set_attn_decode_detail(on ? 1 : 0);
     return check_last();
@@ -227,21 +224,6 @@ RR_API int rr_debug_mlp_schedule(int grid, int inter, int hidden, int slice_kb, 
     *max_items = mlp_schedule(grid, inter, hidden, slice_kb, &items);
     if (!items_out || (size_t)capacity < items.size()) return RR_INVALID_ARGUMENT;
     static_assert(sizeof(MlpItem) == 4 * sizeof(int32_t), "MlpItem layout");
-    memcpy(items_out, items.data(), items.size() * sizeof(MlpItem));
-    return RR_OK;
-}
-
-RR_API int rr_debug_layer_schedule(int grid, int hidden, int inter, int nq, int rows_a3, int s_o, int s3, int slice_kb,
-                                   int has_main, int32_t* items_out, int capacity, int* max_items) {
-    if (grid < 1 || hidden < 64 || hidden % 64 || !max_items) return RR_INVALID_ARGUMENT;
-    if (has_main && (inter < 64 || inter % 64 || nq < 64 || slice_kb < 1)) return RR_INVALID_ARGUMENT;
-    LayerShape sh;
-    sh.hidden = hidden; sh.inter = inter; sh.nq = nq; sh.rowsA3 = rows_a3; sh.s_o = s_o; sh.s3 = s3; sh.slice_kb = slice_kb;
-    sh.has_main = has_main;
-    std::vector<MlpItem> items;
-    *max_items = layer_schedule(grid, sh, &items);
-    if (*max_items < 0) return RR_INVALID_ARGUMENT;
-    if (!items_out || (size_t)capacity < items.size()) return RR_INVALID_ARGUMENT;
     memcpy(items_out, items.data(), items.size() * sizeof(MlpItem));
     return RR_OK;
 }

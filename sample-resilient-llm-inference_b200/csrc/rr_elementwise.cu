@@ -267,7 +267,7 @@ silu_mul_kernel(PartIn gu, __nv_bfloat16* __restrict__ act, int inter) {
     if (c >= inter) return;
     const float4 g = part_load4(gu, row, c);
     const float4 u = part_load4(gu, row, inter + c);
-    auto f = [](float a, float b) { return __fdividef(a, 1.f + __expf(-a)) * b; };   // same formula as silu_mul (rr_gemm_dev.cuh)
+    auto f = [](float a, float b) { return __fdividef(a, 1.f + __expf(-a)) * b; };   // same formula as silu_mul (rr_gemm.cu)
     uint2 o;
     o.x = pack_bf16(f(g.x, u.x), f(g.y, u.y));
     o.y = pack_bf16(f(g.z, u.z), f(g.w, u.w));

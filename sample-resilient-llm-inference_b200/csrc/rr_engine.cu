@@ -9,7 +9,7 @@
 // Layout in HBM (one replica): bf16 weights (caller-owned), KV cache
 // [layer][slot][kv_head][ctx_max][128] bf16 for K and for V, a decode working set of max_batch
 // rows (row b == KV slot b) and a prefill working set of max_prefill_tokens rows.
-// The decode step is a fixed sequence of 9 launches per layer + 4, captured once in a CUDA graph
+// The decode step is a fixed sequence of 6 launches per layer + 4, captured once in a CUDA graph
 // and replayed; per-row metadata (token, position, active flag) lives on the device so replays
 // need no parameter changes.
 #include "rr_kernels.h"
@@ -130,12 +130,6 @@ struct rr_engine {
                                       // GEMM's epilogue applies 1 / rms (RopeEpi)
     float* p_rowss = nullptr;         // [Tmax][pf_parts]
     int pf_parts = 0;
-    bool use_layer = false;           // decode: one persistent dataflow launch per layer between attention kernels (rr_layer.cu)
-    std::vector<LayerPlan> layer;     // [0] = QKV projection of layer 0 only; [1 + l] = layer l (phase 3 = QKV of l + 1 / lm_head)
-    MlpItem* layer_items = nullptr;   // device copies of the three schedules (first | mid | last)
-    unsigned* layer_ctr = nullptr;    // [(L + 1) * layer_ctr_words] dependency counters, zeroed by the first kernel of every step
-    int layer_ctr_words = 0;
-    float *rowss_a = nullptr, *rowss_b = nullptr;   // [Bm][ceil(hidden / 128)] partial sum(x^2) (deferred RMSNorm)
     bool fuse_silu = false;           // wgu interleaved + one gate/up plane: SiLU*mul lives in the GEMM epilogue
     bool fuse_mlp = false;            // decode: gate/up and down GEMMs in one persistent launch (gemm_mlp_tcgen05)
     std::vector<MlpPlan> mlp;         // per layer
@@ -210,9 +204,9 @@ static int pick_splits(int N, int K) {
     return s;
 }
 
-// One engine at a time per device.  The fused MLP kernel and the layer kernel (rr_layer.cu) are persistent grids whose
-// CTAs spin on work of sibling CTAs; two such grids interleaved on one GPU (two engines, two streams) could each hold
-// SMs the other's not-yet-resident CTAs need.  Every path below synchronises its stream before it releases this lock, so
+// One engine at a time per device.  The fused MLP kernel is a persistent grid whose CTAs spin on work of sibling CTAs;
+// two such grids interleaved on one GPU (two engines, two streams) could each hold SMs the other's not-yet-resident CTAs
+// need.  Every path below synchronises its stream before it releases this lock, so
 // engines that share a device alternate at prefill-chunk / decode-step granularity.  (The gateway creates one engine per
 // GPU, so this lock is uncontended there.)
 static std::mutex& device_mutex(int dev) {
@@ -235,23 +229,6 @@ static int enqueue_decode_step(rr_engine* e, cudaStream_t s, uint64_t* n_launch)
     const rr_model_desc& d = e->d;
     const int B = e->Bm, L = d.n_layers;
     uint64_t nl = 0;
-    if (e->use_layer) {
-        // 3 + 2 L + 1 launches: embed, norm (deferred form: xn = bf16(x * gamma), sum(x^2); also zeroes every dependency
-        // counter of the step), QKV_0, then per layer attention + one persistent layer kernel (phase 3 of the last = lm_head)
-        launch_embed(e->d_tok, (const __nv_bfloat16*)e->embed, e->x, B, d.hidden, e->d_slot, s); ++nl;
-        launch_add_rmsnorm(e->x, part_none(), (const __nv_bfloat16*)e->norm_attn[0], e->xn, B, d.hidden, d.rms_eps, s,
-                           e->layer_ctr, (L + 1) * e->layer_ctr_words, e->rowss_b, (d.hidden + 127) / 128); ++nl;
-        if (layer_launch(e->layer[0], s) != RR_OK) return RR_CUDA_ERROR; ++nl;
-        for (int l = 0; l < L; ++l) {
-            launch_decode_attn(e->attn_args[l], s); nl += e->kv_splits > 1 ? 2 : 1;
-            if (layer_launch(e->layer[1 + l], s) != RR_OK) return RR_CUDA_ERROR; ++nl;
-        }
-        launch_argmax(part_f32(e->logits, 1, B, d.vocab), B, d.vocab, e->d_tok, nullptr, e->d_slot, e->d_pos, s); ++nl;
-        if (n_launch) *n_launch = nl;
-        cudaError_t err = cudaGetLastError();
-        if (err != cudaSuccess) { rr::note_cuda_error(err); return RR_CUDA_ERROR; }
-        return RR_OK;
-    }
     launch_embed(e->d_tok, (const __nv_bfloat16*)e->embed, e->x, B, d.hidden, e->d_slot, s); ++nl;
     launch_add_rmsnorm(e->x, part_none(), (const __nv_bfloat16*)e->norm_attn[0], e->xn, B, d.hidden, d.rms_eps, s); ++nl;
     for (int l = 0; l < L; ++l) {
@@ -754,70 +731,6 @@ RR_API int rr_engine_create(const rr_model_desc* desc, const rr_model_weights* w
     // with the earlier row-per-thread epilogue the same fusion LOST 1.4 % (o-proj +35 %).
     e->defer_norm_pf = opts->reserved[3] == 0 && !getenv("RR_NO_DEFER_NORM") && d.hidden % 8 == 0 && e->pf_parts <= 64;
     if (e->defer_norm_pf) TRY(dalloc(e, &e->p_rowss, (size_t)e->Tmax * e->pf_parts));
-    // ---- persistent layer kernel (rr_layer.cu): OFF by default -- reserved[0] = 2 or RR_LAYER_FUSE=1 turns it on.
-    // Measured on B200 (tools/decode_ab.py, same process, alternating): 4.67 ms per decode step against 4.34 ms for the
-    // per-kernel path below.  Under a saturated weight stream every dependent memory round trip costs 2.5 - 4 us (the ring
-    // depth sweep in profiles/r02_layer_kernel_experiment.md), and a dependency counter is 3 - 4 of them (store drain,
-    // release, poll, operand load), while a kernel boundary happens when the memory system has drained.
-    e->use_layer = e->fuse_mlp && (opts->reserved[0] == 2 || getenv("RR_LAYER_FUSE")) && !getenv("RR_NO_LAYER_FUSE");
-    if (e->use_layer) {
-        const int grid = num_sms();
-        const int tiles_h = (d.hidden + 127) / 128, kb_o = (e->nq + 63) / 64;
-        int s_o = grid / tiles_h;                         // one O item per CTA (their epilogues wait for each other)
-        if (s_o > 8) s_o = 8;
-        while (s_o > 1 && kb_o / s_o < 4) --s_o;
-        if (s_o > e->s_o) s_o = e->s_o > 0 ? e->s_o : 1;  // part_o holds e->s_o planes
-        if (s_o < 1 || tiles_h * s_o > grid) e->use_layer = false;
-        if (e->use_layer) {
-            LayerShape sh[3];
-            for (int k = 0; k < 3; ++k) {
-                sh[k].hidden = d.hidden; sh[k].inter = d.inter; sh[k].nq = e->nq; sh[k].s_o = s_o;
-                sh[k].slice_kb = e->mlp_slice_kb; sh[k].has_main = k > 0;
-                sh[k].rowsA3 = k < 2 ? e->nqkv : d.vocab; sh[k].s3 = k < 2 ? e->s_qkv : 1;
-            }
-            std::vector<MlpItem> sched[3];
-            int mx[3];
-            size_t total = 0;
-            for (int k = 0; k < 3; ++k) {
-                mx[k] = layer_schedule(grid, sh[k], &sched[k]);
-                if (mx[k] < 0) { e->use_layer = false; break; }
-                total += sched[k].size();
-            }
-            if (e->use_layer) {
-                TRY(dalloc(e, &e->layer_items, total));
-                size_t off[3], o = 0;
-                for (int k = 0; k < 3; ++k) {
-                    off[k] = o;
-                    TRYC(cudaMemcpy(e->layer_items + o, sched[k].data(), sched[k].size() * sizeof(MlpItem), cudaMemcpyHostToDevice));
-                    o += sched[k].size();
-                }
-                e->layer_ctr_words = (layer_counter_words(sh[1]) + 31) & ~31;
-                TRY(dalloc(e, &e->layer_ctr, (size_t)(L + 1) * e->layer_ctr_words));
-                TRY(dalloc(e, &e->rowss_a, (size_t)B * tiles_h));
-                TRY(dalloc(e, &e->rowss_b, (size_t)B * tiles_h));
-                e->layer.resize(L + 1);
-                for (int i = 0; i <= L; ++i) {
-                    const int l = i - 1;                  // -1: the QKV projection of layer 0 alone
-                    const int k = i == 0 ? 0 : (l + 1 < L ? 1 : 2);
-                    LayerBuffers bf;
-                    memset(&bf, 0, sizeof(bf));
-                    bf.x = e->x; bf.xhat = e->xn; bf.rowss_a = e->rowss_a; bf.rowss_b = e->rowss_b; bf.rows = B; bf.ld_rows = B;
-                    bf.eps = d.rms_eps;
-                    bf.l2_ahead = getenv("RR_LAYER_L2_AHEAD") ? atoi(getenv("RR_LAYER_L2_AHEAD")) : 0;
-                    bf.ring_depth = getenv("RR_LAYER_RING_DEPTH") ? atoi(getenv("RR_LAYER_RING_DEPTH")) : 0;
-                    if (l >= 0) {
-                        bf.wo = e->wo[l]; bf.wgu = e->wgu[l]; bf.wdown = e->wdown[l]; bf.attn_out = e->attn_out; bf.act = e->act;
-                        bf.part_o = e->part_o; bf.part_d = e->part_down; bf.gamma_a = (const __nv_bfloat16*)e->norm_mlp[l];
-                        bf.gamma_b = (const __nv_bfloat16*)(l + 1 < L ? e->norm_attn[l + 1] : e->final_norm);
-                    }
-                    if (k < 2) { bf.w3 = e->wqkv[l + 1]; bf.out3 = e->part_qkv; bf.ldo3 = e->nqkv; }
-                    else { bf.w3 = e->lm_head; bf.out3 = e->logits; bf.ldo3 = d.vocab; }
-                    TRY(layer_plan_init(&e->layer[i], sh[k], bf, e->bn_dec, e->layer_items + off[k], mx[k], grid,
-                                        e->layer_ctr + (size_t)i * e->layer_ctr_words));
-                }
-            }
-        }
-    }
     if (e->fuse_mlp) {
         std::vector<MlpItem> sched;
         const int grid = num_sms();

@@ -18,7 +18,9 @@
 //
 // Replaces: the remote bedrock:InvokeModel call (reference iam/policy.json:8,
 // src/demo_cris.py:233-238) — there is no reference kernel; see DESIGN.md §kernels.
-#include "rr_gemm_dev.cuh"
+#include "rr_ptx.cuh"
+#include "rr_launch.cuh"
+#include "rr_kernels.h"
 
 #include <mutex>
 #include <stdio.h>
@@ -26,6 +28,83 @@
 #include <string.h>
 
 namespace rr {
+
+constexpr int BLOCK_A = 128;   // UMMA M
+constexpr int BLOCK_K = 64;    // 64 bf16 = 128 B = one swizzle row
+constexpr int UMMA_K = 16;
+constexpr int GEMM_THREADS = 192;
+constexpr int GROUP_A = 16;    // raster group: 16 A tiles share the streamed B tiles through L2
+
+// CAP bounds the smem ring.
+template <int BN, int CAP = 8>
+struct GemmCfg {
+    static constexpr int kStageBytesA = BLOCK_A * BLOCK_K * 2;
+    static constexpr int kStageBytesB = BN * BLOCK_K * 2;
+    static constexpr int kStageBytes = kStageBytesA + kStageBytesB;
+    static constexpr int kStagesRaw = (200 * 1024) / kStageBytes;
+    static constexpr int kStages = kStagesRaw > CAP ? CAP : kStagesRaw;
+    static constexpr uint32_t kTmemCols =
+        (2 * BN <= 32) ? 32 : (2 * BN <= 64) ? 64 : (2 * BN <= 128) ? 128 : (2 * BN <= 256) ? 256 : 512;
+    static constexpr int kSmemBytes = kStages * kStageBytes + 1024 /*align slack*/ + 256 /*barriers*/;
+    static constexpr int kSiluStageBytes = 2 * 32 * 64 * 4;   // OUT_TRANSPOSED_SILU: up-row exchange, 2 x [32 cols][64 rows] fp32
+};
+// TMA-store epilogues of the decode orientation (BN <= 64): the planes tile [BN][128] fp32 (one 3-D TMA store per item); the
+// fused MLP kernel aliases it with the up-row exchange (16 KB) + the act tile [BN][64] bf16 of the SiLU epilogue.
+template <int BN>
+constexpr int planes_stage_bytes() { return BN <= 64 ? BN * 128 * 4 : 0; }
+template <int BN>
+constexpr int mlp_stage_bytes() {
+    constexpr int a = planes_stage_bytes<BN>(), b = GemmCfg<BN>::kSiluStageBytes + (BN <= 64 ? BN * 64 * 2 : 0);
+    return a > b ? a : b;
+}
+template <int MODE>
+__host__ __device__ constexpr bool decode_orient() { return MODE == OUT_TRANSPOSED_F32 || MODE == OUT_TRANSPOSED_SILU; }
+template <int BN, int MODE, int CAP = 8>
+constexpr int gemm_smem_bytes() {
+    // SILU (decode): up-row exchange; RESID (prefill): per-warp 32 x 36 fp32 transpose tiles (18 KB) -- same slot
+    return GemmCfg<BN, CAP>::kSmemBytes +
+           (MODE == OUT_TRANSPOSED_SILU ? GemmCfg<BN, CAP>::kSiluStageBytes : MODE == OUT_ROWMAJOR_RESID ? 4 * 32 * 36 * 4 :
+            MODE == OUT_TRANSPOSED_F32 ? planes_stage_bytes<BN>() : 0);
+}
+// SiLU(g) * u.  __fdividef, not `/`: the IEEE division compiles to a convergence-barrier region with a slow-path CALL per element,
+// which serialises the unrolled epilogue loops (2 ulp of fp32 before the bf16 rounding; 0 instead of -1e-36 for g < -87).
+__device__ __forceinline__ float silu_mul(float g, float u) { return __fdividef(g, 1.f + __expf(-g)) * u; }
+
+struct WorkItem {
+    int a_tile, b_tile, z, kb0, kb1;
+};
+
+// Deterministic per-CTA sequence of work items (uniform split-K); every warp role walks the same sequence.
+// (A stream-K split -- k-block units dealt evenly to the SMs regardless of tile boundaries -- was measured in round 1:
+// 4.55 -> 4.92 ms per decode step, the consumers read more planes than the better balance returns; removed.)
+struct WorkSched {
+    int tilesA, tilesB, splits, kblocks, n_work, w;
+
+    __device__ __forceinline__ void init(int rowsA, int rowsB, int K, int splits_, int BN) {
+        tilesA = (rowsA + BLOCK_A - 1) / BLOCK_A;
+        tilesB = (rowsB + BN - 1) / BN;
+        kblocks = (K + BLOCK_K - 1) / BLOCK_K;
+        splits = splits_;
+        n_work = tilesA * tilesB * splits;
+        w = blockIdx.x;
+    }
+    __device__ __forceinline__ bool next(WorkItem& it) {
+        if (w >= n_work) return false;
+        it.z = w % splits;
+        const int q = w / splits;
+        const int per_group = GROUP_A * tilesB;
+        const int g = q / per_group;
+        const int r = q - g * per_group;
+        const int a0 = g * GROUP_A;
+        const int ga = min(GROUP_A, tilesA - a0);
+        it.a_tile = a0 + r % ga;
+        it.b_tile = r / ga;
+        it.kb0 = (int)(((long long)kblocks * it.z) / splits);
+        it.kb1 = (int)(((long long)kblocks * (it.z + 1)) / splits);
+        w += gridDim.x;
+        return true;
+    }
+};
 
 // Epilogue of one work item: TMEM accumulator (this warp's 32 lanes x BN columns at taddr0) -> global memory, in the
 // layout / fusion selected by MODE.  Shared by the 1-CTA kernel, the 2-CTA kernel and (by copy) the chain kernel.

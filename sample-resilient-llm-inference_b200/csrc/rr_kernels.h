@@ -104,59 +104,6 @@ int mlp_plan_init(MlpPlan* p, const void* Wgu, const void* Wd, int inter, int hi
                   unsigned* ready, int slice_kb, int dynamic = 0);
 int mlp_launch(const MlpPlan& p, cudaStream_t st);
 
-// ---- persistent decode layer (rr_layer.cu): O -> (+residual, deferred norm) -> gate/up+SiLU -> down -> (+residual,
-// deferred norm) -> next projection (QKV of the next layer or lm_head), one launch, dependency counters between phases.
-struct LayerShape {
-    int hidden, inter, nq;    // nq = K of the O projection (n_heads * head_dim)
-    int rowsA3;               // phase 3 weight rows (QKV features of the next layer, or vocab); 0 = no phase 3
-    int s_o, s3;              // split-K factors of phase 0 / phase 3
-    int slice_kb;             // k-blocks per down-projection slice
-    int has_main;             // phases 0..2 present (0: phase 3 only -- the QKV projection of layer 0)
-};
-struct LayerBuffers {
-    const void *wo, *wgu, *wdown, *w3;          // weights (wgu 64-row interleaved)
-    const __nv_bfloat16* attn_out;              // [rows, nq]
-    float* x;                                   // [rows, hidden] residual
-    __nv_bfloat16* xhat;                        // [rows, hidden] bf16(x * gamma), un-normalised GEMM operand
-    __nv_bfloat16* act;                         // [rows, inter]
-    float* part_o;                              // [s_o][ld_rows][hidden]
-    float* part_d;                              // [n_slices][ld_rows][hidden] planes of the down projection
-    float* out3;                                // [s3][ld_rows][ldo3]
-    const __nv_bfloat16 *gamma_a, *gamma_b;     // norm weights after O / after down
-    float *rowss_a, *rowss_b;                   // [rows][ceil(hidden / 128)] partial sum(x^2)
-    int rows, ld_rows, ldo3;
-    float eps;
-    int l2_ahead;                               // weight k-blocks prefetched into L2 behind the smem ring while a dependency is awaited
-    int ring_depth;                             // smem ring slots in use (0 = all)
-};
-struct LayerArgs {
-    CUtensorMap tmA[4], tmB[4];
-    float* part_o;
-    float* part_d;
-    float* x;
-    __nv_bfloat16* xhat;
-    __nv_bfloat16* act;
-    float* out3;
-    const __nv_bfloat16 *gamma_a, *gamma_b;
-    float *rowss_a, *rowss_b;
-    int hidden, inter, rows, ld_rows, rowsA3, ldo3, n_part, tiles_h, s_o, n_slices, slice_kb, rows_red_d, l2_ahead, ring_depth;
-    float inv_hidden, eps;
-    const MlpItem* items;     // [grid][max_items]; tile_phase = tile | phase << 16
-    int max_items;
-    unsigned* ctr;            // [2 + 2 * tiles_h + n_slices], zero at launch
-    unsigned o_target, d_target;
-};
-struct LayerPlan {
-    LayerArgs args;
-    int grid, bn;
-};
-int layer_schedule(int grid, const LayerShape& s, std::vector<MlpItem>* items);   // returns max_items, -1: shape unsupported
-int layer_counter_words(const LayerShape& s);
-int layer_red_groups(int grid, int tiles_h);
-int layer_plan_init(LayerPlan* p, const LayerShape& s, const LayerBuffers& b, int bn, const MlpItem* items_dev,
-                    int max_items, int grid, unsigned* ctr);
-int layer_launch(const LayerPlan& p, cudaStream_t st);
-
 // ---- elementwise / normalisation (rr_elementwise.cu) -------------------------------------------
 // `part` inputs are the GEMM outputs: either fp32 split-K partials P[z][row][col] (n_splits >= 1,
 // part_is_bf16 = 0, split stride = split_stride elements) or a single bf16 matrix.
@@ -171,7 +118,7 @@ struct PartIn {
 void launch_embed(const int32_t* ids, const __nv_bfloat16* table, float* x, int rows, int hidden,
                   const int32_t* row_active, cudaStream_t st);
 // x[row] (+)= sum_z part[z][row]; xn[row] = rmsnorm(x[row]) * w   (part.ptr may be null: norm only)
-// `zero` (optional): zero_n dependency counters reset by the kernel (fused MLP kernel / layer kernels that follow it).
+// `zero` (optional): zero_n dependency counters reset by the kernel (the fused MLP kernel that follows it).
 // `rowss_out` (optional, deferred norm): write xn = bf16(x * w) UN-normalised and rowss_out[row][0] = sum(x^2),
 // rowss_out[row][1 .. n_part_out) = 0 -- the layout the OUT_ROWMAJOR_RESID epilogue produces (RopeEpi).
 void launch_add_rmsnorm(float* x, PartIn part, const __nv_bfloat16* w, __nv_bfloat16* xn, int rows,

@@ -19,13 +19,12 @@ __device__ __forceinline__ void griddep_launch() { asm volatile("griddepcontrol.
 // (kernel id, globaltimer at start, after griddepcontrol.wait, at end) into a device buffer; rr_debug_trace_*.
 // Each translation unit owns its copy of the pointer (no -rdc); rr_api.cu sets them all.
 static __device__ unsigned long long* rr_trace_ptr = nullptr;
-static __device__ int rr_trace_detail = 0;      // 1: also per-item marks of sample CTAs (trace_mark_cta), a few % slower
+static __device__ int rr_trace_detail = 0;      // 1: also per-item marks of sample CTAs (trace_mark_fixed / trace_mark_at), a few % slower
 static inline void rr_trace_set_local(unsigned long long* p) { cudaMemcpyToSymbol(rr_trace_ptr, &p, sizeof(p)); }
 static inline void rr_trace_set_detail_local(int on) { cudaMemcpyToSymbol(rr_trace_detail, &on, sizeof(on)); }
 enum TraceId { TR_GEMM_DEC = 1, TR_GEMM_PF = 2, TR_ATTN_DEC = 3, TR_ATTN_PF = 4, TR_NORM = 5, TR_ROPE = 6,
                TR_SILU = 7, TR_EMBED = 8, TR_ARGMAX = 9, TR_COMBINE = 10, TR_MISC = 11,
-               TR_LAYER_PH0 = 12,
-               TR_MLP_MARK = 50, TR_ATTN_MARK = 80, TR_GEMM_MARK = 100 };  // + k: sample CTAs of the fused MLP kernel (tools/trace_mlp.py)  // + k: sample CTAs of the layer kernel finished an item (0 O, 1 gate/up, 2 down, 3 reduce, 4 next)
+               TR_MLP_MARK = 50, TR_ATTN_MARK = 80, TR_GEMM_MARK = 100 };  // + k: sample CTAs of the fused MLP kernel (tools/trace_mlp.py)
 __device__ __forceinline__ unsigned long long rr_gtimer() {
     unsigned long long t;
     asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
@@ -44,30 +43,11 @@ __device__ __forceinline__ int trace_begin(int kid) {
 __device__ __forceinline__ void trace_dep(int slot) {
     if (slot >= 0) rr_trace_ptr[4 + 4 * slot] = rr_gtimer();
 }
-// single-thread marker from inside a kernel (caller guarantees one calling thread in CTA 0)
-__device__ __forceinline__ void trace_mark(int kid) {
-    unsigned long long* p = rr_trace_ptr;
-    if (p == nullptr || (blockIdx.x | blockIdx.y | blockIdx.z) != 0) return;
-    const int slot = (int)atomicAdd(p, 1ull);
-    if (slot >= (int)p[1]) return;
-    const unsigned long long t = rr_gtimer();
-    p[2 + 4 * slot] = (unsigned long long)kid;
-    p[3 + 4 * slot] = t; p[4 + 4 * slot] = t; p[5 + 4 * slot] = t;
-}
-// marker from a few sample CTAs (0, 37, 74, 111, ...): kid in the low byte, CTA index above it
-__device__ __forceinline__ void trace_mark_cta(int kid) {
-    unsigned long long* p = rr_trace_ptr;
-    if (p == nullptr || rr_trace_detail == 0 || blockIdx.x % 37 != 0) return;
-    const int slot = (int)atomicAdd(p, 1ull);
-    if (slot >= (int)p[1]) return;
-    const unsigned long long t = rr_gtimer();
-    p[2 + 4 * slot] = (unsigned long long)(kid | ((int)blockIdx.x << 8));
-    p[3 + 4 * slot] = t; p[4 + 4 * slot] = t; p[5 + 4 * slot] = t;
-}
-// Same sample CTAs, but NO atomic: the slot is a fixed function of (sample CTA, idx) at the END of the buffer, so the marking
-// thread never waits for a memory round trip (an atomicAdd with a result costs 2-4 us under a saturated weight stream and
-// would distort exactly the latencies being measured).  idx < 192 per CTA; rr_debug_trace_stop returns the whole buffer
-// while detail marks are on and the reader drops the empty rows.
+// Marker from a few sample CTAs (0, 37, 74, 111, ...): kid in the low byte, CTA index above it.  NO atomic: the slot is a
+// fixed function of (sample CTA, idx) at the END of the buffer, so the marking thread never waits for a memory round trip
+// (an atomicAdd with a result costs 2-4 us under a saturated weight stream and would distort exactly the latencies being
+// measured).  idx < 192 per CTA; rr_debug_trace_stop returns the whole buffer while detail marks are on and the reader
+// drops the empty rows.
 __device__ __forceinline__ void trace_mark_fixed(int kid, int idx) {
     unsigned long long* p = rr_trace_ptr;
     if (p == nullptr || rr_trace_detail == 0 || blockIdx.x % 37 != 0 || idx >= 192) return;

@@ -1,7 +1,7 @@
 // rr_ptx.cuh — thin inline-PTX wrappers for sm_100a (Blackwell B200).
 //
-// mbarrier, TMA (cp.async.bulk.tensor), tcgen05 (alloc / mma / commit / ld),
-// cp.async and a few cache-hinted vector loads. Nothing here is portable: this
+// mbarrier, TMA (cp.async.bulk.tensor), tcgen05 (alloc / mma / commit / ld)
+// and a few cache-hinted vector loads. Nothing here is portable: this
 // file only compiles for compute_100a.
 #pragma once
 #include <cuda_runtime.h>
@@ -13,12 +13,6 @@ namespace rr {
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {
     return static_cast<uint32_t>(__cvta_generic_to_shared(p));
-}
-
-__device__ __forceinline__ uint32_t lane_id() {
-    uint32_t l;
-    asm volatile("mov.u32 %0, %%laneid;" : "=r"(l));
-    return l;
 }
 
 // One lane of a fully-converged warp is elected; returns true in that lane.
@@ -103,12 +97,6 @@ __device__ __forceinline__ void tma_load_2d_hint(void* smem_dst, const CUtensorM
         ::"r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar)),
         "r"(c0), "r"(c1), "l"(policy)
         : "memory");
-}
-// L2 prefetch of one tile (no shared-memory destination, no barrier).
-__device__ __forceinline__ void tma_prefetch_l2_2d(const CUtensorMap* m, int32_t c0, int32_t c1) {
-    asm volatile("cp.async.bulk.prefetch.tensor.2d.L2.global.tile [%0, {%1, %2}];"
-                 ::"l"(reinterpret_cast<uint64_t>(m)), "r"(c0), "r"(c1)
-                 : "memory");
 }
 // ---- TMA stores (shared -> global, bulk async-group completion)
 __device__ __forceinline__ void tma_store_2d(const CUtensorMap* m, const void* smem_src, int32_t c0, int32_t c1) {
@@ -230,23 +218,6 @@ __host__ __device__ constexpr uint32_t umma_idesc_bf16_f32(uint32_t M, uint32_t 
            | (1u << 10)              // b_format  = BF16
            | ((N >> 3) << 17)        // n_dim
            | ((M >> 4) << 24);       // m_dim
-}
-
-// ---------------------------------------------------------------- cp.async (LDGSTS)
-__device__ __forceinline__ void cp_async_16(void* smem_dst, const void* gsrc) {
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(smem_u32(smem_dst)), "l"(gsrc)
-                 : "memory");
-}
-__device__ __forceinline__ void cp_async_16_zfill(void* smem_dst, const void* gsrc, bool valid) {
-    int sz = valid ? 16 : 0;
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(smem_u32(smem_dst)),
-                 "l"(gsrc), "r"(sz)
-                 : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void cp_async_wait() {
-    asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory");
 }
 
 // ---------------------------------------------------------------- misc loads

@@ -47,7 +47,7 @@ def _p(a: np.ndarray):
 class Engine:
     def __init__(self, weights: Weights, device: int = 0, max_batch: int = 64, ctx_max: int = 1024,
                  max_prefill_tokens: int = 8192, use_cuda_graph: bool = True,
-                 fail_prob: float = 0.0, fail_seed: int = 0, fuse_silu: bool = True, fuse_layer: bool = False,
+                 fail_prob: float = 0.0, fail_seed: int = 0, fuse_silu: bool = True,
                  fuse_mlp: bool = True, defer_norm: bool = True):
         if not torch.cuda.is_available():
             raise RuntimeError("rr_b200.Engine needs a CUDA device (no CPU fallback)")
@@ -88,7 +88,7 @@ class Engine:
                                weights.final_norm.data_ptr(), *self._arrs, 1 if self.fuse_silu else 0, 0)
         opts = _lib.EngineOpts(device, max_batch, ctx_max, max_prefill_tokens,
                                1 if use_cuda_graph else 0, fail_seed, fail_prob,
-                               (C.c_int32 * 4)(2 if fuse_layer else 1, 0, 0 if fuse_mlp else 1, 0 if defer_norm else 1))
+                               (C.c_int32 * 4)(0, 0, 0 if fuse_mlp else 1, 0 if defer_norm else 1))
         torch.cuda.synchronize(device)   # weights were produced on torch's stream
         self._h = C.c_void_p()
         _lib.check(_lib.lib.rr_engine_create(C.byref(desc), C.byref(mw), C.byref(opts),

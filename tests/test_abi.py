@@ -105,103 +105,3 @@ def test_fused_mlp_schedule_is_a_partition_and_deadlock_free(grid, inter, hidden
     assert sum(loads) == total
     if grid >= 64 and total // grid >= 100:                    # the production shapes: within 15 % of the mean
         assert max(loads) <= 1.15 * total / grid + slice_kb
-
-
-@pytest.mark.parametrize("grid,hidden,inter,nq,rows3,s_o,s3,slice_kb,has_main", [
-    (148, 4096, 14336, 4096, 6144, 4, 3, 28, 1),        # Llama-3-8B / Mistral-7B middle layer
-    (148, 4096, 14336, 4096, 128256, 4, 1, 28, 1),      # last layer: phase 3 = lm_head
-    (148, 4096, 14336, 4096, 6144, 4, 3, 28, 0),        # QKV projection of layer 0 alone
-    (148, 3072, 8192, 3072, 9216, 6, 2, 16, 1),         # Phi-3-mini
-    (148, 1024, 2816, 1024, 1536, 4, 2, 15, 1),         # small
-    (132, 768, 2048, 768, 1152, 3, 1, 16, 1),           # small96 on a smaller grid
-])
-def test_layer_schedule_is_a_partition_and_the_dataflow_terminates(grid, hidden, inter, nq, rows3, s_o, s3, slice_kb, has_main):
-    """Host logic of the persistent decode layer kernel (csrc/rr_layer.cu, layer_schedule).  Every item appears exactly
-    once; each CTA's list is ordered by phase (O, gate/up, down, reduce, next); O items are first and at most one per CTA
-    (their epilogues wait for each other).  Then the dependency rules of the kernel are replayed on the lists (a CTA finishes an item only
-    when the counters it spins on have reached their targets): the replay must drain every list, i.e. no wait cycle."""
-    import numpy as np
-    from rr_b200 import _lib as lib
-    mx = C.c_int32()
-    cap = grid * 256
-    buf = np.full((cap, 4), -7, dtype=np.int32)
-    rc = lib.lib.rr_debug_layer_schedule(grid, hidden, inter, nq, rows3, s_o, s3, slice_kb, has_main,
-                                         buf.ctypes.data_as(C.POINTER(C.c_int32)), cap, C.byref(mx))
-    assert rc == 0 and 1 <= mx.value <= 256
-    items = buf[: grid * mx.value].reshape(grid, mx.value, 4)
-    tiles_h, tiles_gu, tiles3 = (hidden + 127) // 128, 2 * inter // 128, (rows3 + 127) // 128
-    kb_h, kb_o, kb_d = (hidden + 63) // 64, (nq + 63) // 64, inter // 64
-    n_slices = (kb_d + slice_kb - 1) // slice_kb
-    n_rq = grid // tiles_h
-    n_rq = 1 if n_rq < 1 else (8 if n_rq > 8 else (4 if n_rq >= 4 else n_rq))          # layer_red_groups()
-    ORDER = {0: 0, 1: 1, 2: 2, 4: 3, 3: 4}                        # list order of the phases (4 = reduce items)
-    lists, seen, loads = [], set(), []
-    for c in range(grid):
-        lst, ended, key_prev, load = [], False, -1, 0
-        for tp, k0, k1, z in items[c]:
-            if tp < 0:
-                ended = True
-                continue
-            assert not ended
-            ph, tile = int(tp) >> 16, int(tp) & 0xFFFF
-            assert ORDER[ph] >= key_prev, (c, ph, key_prev)        # ordered by phase
-            key_prev = ORDER[ph]
-            assert (ph, tile, int(z)) not in seen
-            seen.add((ph, tile, int(z)))
-            if ph == 0:
-                assert not lst and tile < tiles_h and 0 <= z < s_o        # first item of its CTA
-                assert (k0, k1) == (kb_o * z // s_o, kb_o * (z + 1) // s_o)
-            elif ph == 1:
-                assert tile < tiles_gu and (k0, k1) == (0, kb_h)
-            elif ph == 2:
-                assert tile < tiles_h and k0 == z * slice_kb and k1 == min(kb_d, k0 + slice_kb)
-            elif ph == 4:
-                assert tile < tiles_h and 0 <= z < n_rq and k0 == k1
-            else:
-                assert ph == 3 and tile < tiles3 and (k0, k1) == (kb_h * z // s3, kb_h * (z + 1) // s3)
-            lst.append((ph, tile, int(z), int(k1 - k0)))
-            load += int(k1 - k0)
-        lists.append(lst)
-        loads.append(load)
-    want = tiles3 * s3 + (tiles_h * s_o + tiles_gu + tiles_h * n_slices + tiles_h * n_rq if has_main else 0)
-    assert len(seen) == want
-    # ---- replay the dependency rules (rr_layer.cu): arr_o, cnt_o, ready_gu[slice], arr_d[tile], cnt_d
-    cur = [0] * grid
-    arrived = [False] * grid                 # O item of this CTA has stored its planes (no dependency besides attention)
-    arr_o, arr_d, ready = [0] * tiles_h, [0] * tiles_h, [0] * n_slices
-    cnt_o = cnt_d = 0
-    o_target, d_target = (tiles_h * s_o, tiles_h * n_rq) if has_main else (0, 0)
-    progress = True
-    while progress:
-        progress = False
-        for c in range(grid):
-            while cur[c] < len(lists[c]):
-                ph, tile, z, nkb = lists[c][cur[c]]
-                if ph == 0:
-                    if not arrived[c]:
-                        arrived[c] = True; arr_o[tile] += 1; progress = True
-                    if arr_o[tile] < s_o:
-                        break
-                    cnt_o += 1
-                elif ph == 1:
-                    if cnt_o < o_target:
-                        break
-                    ready[tile // slice_kb] += 1
-                elif ph == 2:
-                    if ready[z] < nkb:
-                        break
-                    arr_d[tile] += 1
-                elif ph == 4:
-                    if arr_d[tile] < n_slices:
-                        break
-                    cnt_d += 1
-                else:
-                    if cnt_d < d_target:
-                        break
-                cur[c] += 1
-                progress = True
-    assert all(cur[c] == len(lists[c]) for c in range(grid)), "dependency replay stalled: wait cycle in the schedule"
-    assert cnt_d == d_target and cnt_o == o_target
-    total = sum(loads)
-    if grid >= 64 and total // grid >= 100:
-        assert max(loads) <= 1.2 * total / grid + 64
